@@ -6,7 +6,7 @@ triples per GPU; ~98 % valid, ~1 % single-bit corruptions, ~1 % adversarial enco
 (rusty_kaspa_b200/workload.py).  One "step" = one pass of the verify kernel over the rank's batch,
 followed (N > 1) by the NCCL all-gather of the per-shard validity bitmaps.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n ITEMS]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--n ITEMS] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun, one rank per GPU; shards are independent (weak scaling: every rank
 verifies its own 1 Mi triples), the only collective is the bitmap all-gather.
@@ -38,6 +38,21 @@ N_DEFAULT = 1 << 20
 ALG_BYTES_PER_VERIFY = 129  # 32 pk + 32 msg + 64 sig read, 1 status byte written (SURVEY.md §8d)
 METRIC = "schnorr_sig_verifies_per_sec"
 UNIT = "verifies/s"
+DUMP_MAX_BYTES = 60 << 20  # --dump-outputs: under 64 MB in all with the .npy headers
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes each array as out_dir/<name>.npy in float32, so that two builds run with the same arguments (hence the
+    same seeded inputs) can be compared output for output.  Beyond DUMP_MAX_BYTES in all, every array is cut to the same fixed,
+    seeded sample of its elements (sorted indices from default_rng(0)), so the files stay comparable between runs."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(a.size for a in arrays.values())
+    for name, a in arrays.items():
+        a = a.reshape(-1)
+        k = min(a.size, a.size * (DUMP_MAX_BYTES // 4) // total)
+        if k < a.size:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, k, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -239,6 +254,8 @@ def run_reference(args, rank, world):
         dt, st = oracle_verify(lib, pk, msg, sig, threads)
         total += dt
     assert int((st == 1).sum()) == int((kind == 0).sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"status": st})
     value = n * args.steps / total
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
             "ms_per_step": total / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "u64 limbs (256-bit modular integer)",
@@ -814,6 +831,8 @@ def run_ours(args, rank, world, local_rank):
         st = dst.cpu().numpy()
         assert int((st == 1).sum()) == expected_valid, "GPU verdicts disagree with the generator's ground truth"
         assert not (st[kind != 0] == 1).any()
+        if args.dump_outputs and rank == 0:  # the last timed step's verdicts and the bitmap every rank ends up with
+            dump_outputs(args.dump_outputs, {"status": st, "bitmap": (gathered if world > 1 else dbm).cpu().numpy()})
         mine = np.zeros(nbm, dtype=np.uint8)
         pb = np.packbits((st == 1).astype(np.uint8), bitorder="little")
         mine[:len(pb)] = pb
@@ -977,7 +996,10 @@ def main():
     ap.add_argument("--replay-blocks", type=int, default=10000, help="blocks of the DAG-replay leg (BASELINE configs[2]: 10k blocks; 0 = skip)")
     ap.add_argument("--replay-window", type=int, default=1024, help="blocks per kgv_replay_window call")
     ap.add_argument("--tx-window", type=int, default=32768, help="transactions in the secondary txs-validated/s measurement (0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs (per-triple verdicts, validity bitmap) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     _quiet_stdout()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -4,7 +4,7 @@
 Run in the build container (needs /root/reference; the GPU box does not have it):
     python tests/golden/make_golden.py
 Outputs (committed): tests/golden/{hashers,tx_hashing,sighash,check_scripts_kat,muhash}.json, simpa_goref_1060.json.gz,
-simpa_goref_pruning_5000.json.gz, script_tests.json.gz
+simpa_goref_1060_blocks.json.gz (the raw dump, unconverted), simpa_goref_pruning_5000.json.xz, script_tests.json.gz
 
 Everything is parsed out of the reference's Rust test sources / test data at run time — nothing is
 retyped by hand — and each fixture records the file:line range it came from:
@@ -20,8 +20,10 @@ retyped by hand — and each fixture records the file:line range it came from:
 """
 import gzip
 import json
+import lzma
 import os
 import re
+import shutil
 import sys
 
 REF = "/root/reference"
@@ -36,6 +38,9 @@ def read(rel):
 def dump(name, obj):
     if name.endswith(".gz"):
         with gzip.GzipFile(os.path.join(OUT, name), "wb", mtime=0) as f:
+            f.write(json.dumps(obj, separators=(",", ":")).encode())
+    elif name.endswith(".xz"):
+        with lzma.open(os.path.join(OUT, name), "wb", preset=9 | lzma.PRESET_EXTREME) as f:
             f.write(json.dumps(obj, separators=(",", ":")).encode())
     else:
         with open(os.path.join(OUT, name), "w") as f:
@@ -160,7 +165,7 @@ def check_scripts_kat():
 
 
 # ------------------------------------------------------------------------------------ simpa DAG fixture
-def _simpa_fixture(rel, out_name, note_extra=""):
+def _simpa_fixture(rel, out_name, note_extra="", keep_hash_merkle_root=True):
     with gzip.open(os.path.join(REF, rel), "rt") as f:
         lines = f.read().splitlines()
     params = json.loads(lines[0])
@@ -180,6 +185,8 @@ def _simpa_fixture(rel, out_name, note_extra=""):
                            "accepted_id_merkle_root": h["acceptedIdMerkleRoot"], "utxo_commitment": h["utxoCommitment"],
                            "parents": h["parentsByLevel"][0] if h["parentsByLevel"] else [], "blue_work": h["blueWork"], "blue_score": h["blueScore"],
                            "transactions": [conv_tx(t) for t in b["transactions"]]})
+        if not keep_hash_merkle_root:
+            del out_blocks[-1]["hash_merkle_root"]
     dump(out_name, {"source": rel, "coinbase_maturity": params.get("blockrate", {}).get("coinbase_maturity", params.get("coinbase_maturity")),
                     "storage_mass_parameter": params.get("storage_mass_parameter"),
                     "note": "simpa-generated DAG (simpa/generate-json-tests-data.sh); the reference's json_test replays it and asserts "
@@ -191,9 +198,15 @@ def _simpa_fixture(rel, out_name, note_extra=""):
 
 
 def simpa_fixture():
-    _simpa_fixture("testing/integration/testdata/dags_for_json_tests/goref-1060-tx-265-blocks/blocks.json.gz", "simpa_goref_1060.json.gz")
-    _simpa_fixture("testing/integration/testdata/dags_for_json_tests/goref_custom_pruning_depth/blocks.json.gz", "simpa_goref_pruning_5000.json.gz",
-                   "  5 001 blocks, 4 790 signed single-input transactions (json_test `goref_custom_pruning_depth_test`).")
+    src_1060 = "testing/integration/testdata/dags_for_json_tests/goref-1060-tx-265-blocks/blocks.json.gz"
+    _simpa_fixture(src_1060, "simpa_goref_1060.json.gz")
+    # the same DAG in the reference's own dump format, for the rusty_kaspa_b200.blocks_json reader test
+    shutil.copyfile(os.path.join(REF, src_1060), os.path.join(OUT, "simpa_goref_1060_blocks.json.gz"))
+    print("wrote simpa_goref_1060_blocks.json.gz")
+    # hashMerkleRoot is left out of this one (no test reads it for this DAG): with xz that keeps the file under 1 MB
+    _simpa_fixture("testing/integration/testdata/dags_for_json_tests/goref_custom_pruning_depth/blocks.json.gz", "simpa_goref_pruning_5000.json.xz",
+                   "  5 001 blocks, 4 790 signed single-input transactions (json_test `goref_custom_pruning_depth_test`); hashMerkleRoot not kept.",
+                   keep_hash_merkle_root=False)
 
 
 # ------------------------------------------------------------------------------------ script engine rows

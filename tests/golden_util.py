@@ -1,6 +1,7 @@
 """Helpers shared by the golden-vector tests: fixture loading and the tx dict <-> bytes conventions."""
 import gzip
 import json
+import lzma
 import os
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -8,8 +9,8 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 def load(name):
     path = os.path.join(GOLDEN, name)
-    if name.endswith(".gz"):
-        with gzip.open(path, "rt") as f:
+    if name.endswith(".gz") or name.endswith(".xz"):
+        with (gzip.open if name.endswith(".gz") else lzma.open)(path, "rt") as f:
             return json.load(f)
     with open(path) as f:
         return json.load(f)

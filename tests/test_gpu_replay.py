@@ -69,7 +69,7 @@ def test_multiset_hash_follows_the_utxo_set(gpu_ctx):
     r.close()
 
 
-@pytest.mark.parametrize("fixture,check_every", [("simpa_goref_1060.json.gz", 1), ("simpa_goref_pruning_5000.json.gz", 64)])
+@pytest.mark.parametrize("fixture,check_every", [("simpa_goref_1060.json.gz", 1), ("simpa_goref_pruning_5000.json.xz", 64)])
 def test_virtual_chain_of_the_simpa_dag_reproduces_the_reference_headers(gpu_ctx, fixture, check_every):
     """The reference's simpa DAG fixture replayed on the GPU along its virtual selected-parent chain, mergeset by mergeset in consensus
     order (golden_util.simpa_dag_replay_plan): kgv_validate_txs against the GPU UTXO table (selected parent: SkipScriptChecks, the
@@ -262,7 +262,7 @@ def test_window_with_sibling_duplicates_double_spends_and_rejected_creators(gpu_
     ost.close()
 
 
-@pytest.mark.parametrize("fixture", ["simpa_goref_1060.json.gz", "simpa_goref_pruning_5000.json.gz"])
+@pytest.mark.parametrize("fixture", ["simpa_goref_1060.json.gz", "simpa_goref_pruning_5000.json.xz"])
 def test_whole_virtual_chain_as_one_replay_window_reproduces_every_header_commitment(gpu_ctx, fixture):
     """The reference's simpa DAG fixtures, their whole virtual chain as ONE kgv_replay_window call: per chain block the merged blocks in consensus
     order with the chain block's daa score, the selected parent flagged ACCEPT_COINBASE | SKIP_SCRIPTS (utxo_validation.rs:116-140).  Then

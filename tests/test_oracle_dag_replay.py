@@ -89,5 +89,5 @@ def test_every_header_commitment_of_the_simpa_dag(oracle):
 
 def test_virtual_chain_of_the_5000_block_dag(oracle):
     """goref_custom_pruning_depth (5 001 blocks, 4 790 signed transactions): the 1 665 blocks of the virtual selected-parent chain"""
-    n, accepted = _replay(oracle, "simpa_goref_pruning_5000.json.gz", None, chain_only=True)
+    n, accepted = _replay(oracle, "simpa_goref_pruning_5000.json.xz", None, chain_only=True)
     assert n > 1500 and accepted > 4500

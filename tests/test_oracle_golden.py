@@ -111,16 +111,13 @@ def test_hash_merkle_roots_of_the_simpa_dag(oracle):
 
 
 def test_blocks_json_reader_matches_the_committed_fixture():
-    """rusty_kaspa_b200.blocks_json reads the reference's own dump format; on the build container (which has /root/reference) its
-    output must equal the committed conversion of the same file (tests/golden/simpa_goref_1060.json.gz)."""
+    """rusty_kaspa_b200.blocks_json reads the reference's own dump format: its output for the reference's goref-1060 dump
+    (tests/golden/simpa_goref_1060_blocks.json.gz, stored as the reference wrote it) must equal the committed conversion of the same
+    file (tests/golden/simpa_goref_1060.json.gz)."""
     import os
-    import pytest
-    from golden_util import load, tx_from_json
+    from golden_util import GOLDEN, load, tx_from_json
     from rusty_kaspa_b200.blocks_json import load_blocks_json
-    src = "/root/reference/testing/integration/testdata/dags_for_json_tests/goref-1060-tx-265-blocks/blocks.json.gz"
-    if not os.path.exists(src):
-        pytest.skip("reference tree not present (GPU box)")
-    params, blocks = load_blocks_json(src)
+    params, blocks = load_blocks_json(os.path.join(GOLDEN, "simpa_goref_1060_blocks.json.gz"))
     fx = load("simpa_goref_1060.json.gz")
     assert len(blocks) == len(fx["blocks"]) == 266
     for b, g in zip(blocks, fx["blocks"]):
